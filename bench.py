@@ -439,6 +439,34 @@ def timed_train(module, cfg, rngs_host, warmup, dev, world, local_rank, profile=
     return float(t.item()), int(launches), clocks, out, prof, eng
 
 
+DUMP_MAX_ELEMS = 1 << 20     # per array; a larger output is dumped as a fixed, seeded sample of its flattened entries
+DUMP_MAX_BYTES = 64 << 20    # all files of one --dump-outputs together
+
+
+def dump_outputs(out_dir, out):
+    """Writes what train() returned after its last update as <out_dir>/<name>.npy, so that two builds run with the
+    same arguments can be compared output for output: the last column of every metric, the final parameters, RAdam
+    moments, normalisation statistics, observations, env state and runner key.  Floating-point arrays are written as
+    float32, integer ones (packed observation words, env state, counters) as float64, which holds them exactly.  An
+    array of more than DUMP_MAX_ELEMS entries keeps the flattened entries at the sorted positions
+    np.random.default_rng(0).choice(size, DUMP_MAX_ELEMS, replace=False): the same positions on every run."""
+    train_state, (obs, env_state), _, rng = out["runner_state"]
+    arrays = {f"metrics_{k.replace('/', '_')}": v[:, -1] for k, v in out["metrics"].items()}
+    arrays.update(params=train_state.params_flat, radam_mu=train_state.opt_state.mu,
+                  radam_nu=train_state.opt_state.nu, batch_stats=train_state.batch_stats_flat,
+                  obs_packed=obs, env_state=env_state, rng=rng)
+    os.makedirs(out_dir, exist_ok=True)
+    total = 0
+    for name, t in arrays.items():
+        a = t.cpu().numpy().reshape(-1)
+        a = a.astype(np.float32 if np.issubdtype(a.dtype, np.floating) else np.float64)
+        if a.size > DUMP_MAX_ELEMS:
+            a = a[np.sort(np.random.default_rng(0).choice(a.size, DUMP_MAX_ELEMS, replace=False))]
+        total += a.nbytes
+        assert total <= DUMP_MAX_BYTES, f"--dump-outputs would exceed {DUMP_MAX_BYTES} bytes"
+        np.save(os.path.join(out_dir, f"{name}.npy"), a)
+
+
 E2E_PARTS = {}     # wall-clock split of the last e2e_train call (this rank)
 
 
@@ -511,6 +539,8 @@ def run_gpu(args, rank, world, local_rank):
     graph_used = bool(eng.graph_captured)
     env_steps = seeds_total * args.steps * NUM_STEPS * args.envs
     value = env_steps / (ms_max / 1e3)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out)
 
     # ---- (2) e2e through the public API from host buffers
     e2e_s, h2d, d2h = e2e_train(pqn_minatar, base_config(args.steps, num_envs=args.envs), rngs_host, dev, world, shard=shard)
@@ -681,7 +711,14 @@ def main():
                          "all-reduce the gradient once per minibatch step; auto: envs when --seeds < #GPUs")
     ap.add_argument("--with-eval", action="store_true",
                     help="TEST_DURING_TRAINING=True with the reference's cadence (SURVEY 8(d): report both)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed updates, write what train() returned after the last one as DIR/<name>.npy "
+                         "(headline config; with several GPUs, rank 0's seeds)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.impl != "b200" or args.config != "headline"):
+        ap.error("--dump-outputs is implemented for the headline config of the CUDA path")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
