@@ -43,10 +43,11 @@ extern "C" {
 #define PQN_ENV_SEAQUEST 4        /* "Seaquest-MinAtar" */
 #define PQN_ENV_CARTPOLE 16       /* "CartPole-v1" */
 #define PQN_ENV_ACROBOT 17        /* "Acrobot-v1" */
+#define PQN_ENV_MEMORY_CHAIN 32   /* "MemoryChain-bsuite" (num_bits = 1) */
 
 typedef struct pqn_env_info_t {
   int32_t state_words;      /* uint32 words per env in the SoA state block (incl. 5 LogWrapper words) */
-  int32_t obs_dim;          /* flattened observation length (400 for Breakout, 4 CartPole, 6 Acrobot) */
+  int32_t obs_dim;          /* flattened observation length (400 for Breakout, 4 CartPole, 6 Acrobot, 3 MemoryChain) */
   int32_t obs_shape[3];     /* (H, W, C) for MinAtar, (D, 1, 1) for classic control */
   int32_t num_actions;      /* env.action_space(params).n  — pqn_minatar.py:151 */
   int32_t max_steps;        /* env_params.max_steps_in_episode default — pqn_minatar.py:105 */
@@ -99,13 +100,26 @@ int pqn_permutation(const uint32_t* keys, int64_t n, int32_t S, int rng_mode, in
  * info outputs may be NULL.  max_steps <= 0 selects the env default. */
 int pqn_env_reset(int env_id, const uint32_t* keys, uint32_t* state, float* obs, int64_t N, int max_steps,
                   int rng_mode, void* stream);
+/* gymnax EnvParams beyond the step limit.  max_steps <= 0 selects the env default (max_steps_in_episode).
+ * memory_length: MemoryChain's memory_length (>= 1; 5 is gymnax's default, which pqn_env_reset uses); ignored by
+ * envs without that parameter.  MemoryChain keeps it in its state, so pqn_env_step / pqn_rollout_act_step and their
+ * auto-resets use the value the envs were reset with. */
+typedef struct pqn_env_params_t {
+  int32_t max_steps;
+  int32_t memory_length;
+} pqn_env_params_t;
+/* pqn_env_reset with explicit env parameters (params_host: a host pointer, not NULL).  Returns PQN_E_INVALID for
+ * memory_length < 1 on an env that has the parameter. */
+int pqn_env_reset_params(int env_id, const uint32_t* keys, uint32_t* state, float* obs, int64_t N,
+                         const pqn_env_params_t* params_host, int rng_mode, void* stream);
 int pqn_env_step(int env_id, const uint32_t* keys, uint32_t* state, const int32_t* action, float* obs,
                  float* reward, uint8_t* done, float* info_discount, float* info_returned_episode_returns,
                  int32_t* info_returned_episode_lengths, int32_t* info_timestep, int64_t N, int max_steps,
                  int rng_mode, void* stream);
 /* current observation of `state` as packed bits (binary_obs envs): uint32[N][packed_obs_words] */
 int pqn_env_obs_packed(int env_id, const uint32_t* state, uint32_t* obs_packed, int64_t N, void* stream);
-/* current observation of `state` as float32[N][obs_dim] */
+/* current observation of `state` as float32[N][obs_dim] (MemoryChain: the observation its last reset or step
+ * returned, i.e. get_obs of the state before that step, as bsuite's step emits it) */
 int pqn_env_obs(int env_id, const uint32_t* state, float* obs, int64_t N, void* stream);
 
 /* ---- epsilon-greedy (eps_greedy_exploration, pqn_minatar.py:115-128,194-196) */

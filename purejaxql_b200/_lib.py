@@ -20,6 +20,10 @@ class EnvInfo(Structure):
                 ("packed_obs_words", c_int32)]
 
 
+class EnvParams(Structure):
+    _fields_ = [("max_steps", c_int32), ("memory_length", c_int32)]
+
+
 class NetDesc(Structure):
     _fields_ = [("kind", c_int32), ("in_c", c_int32), ("hidden", c_int32), ("layers", c_int32),
                 ("num_actions", c_int32), ("norm_type", c_int32), ("norm_input", c_int32)]
@@ -56,6 +60,8 @@ _SIGS = {
     "pqn_permutation_workspace_bytes": (c_int64, [c_int64, c_int]),
     "pqn_permutation": (c_int, [c_void_p, c_int64, c_int, c_int, c_void_p, c_int64, c_void_p, c_void_p]),
     "pqn_env_reset": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p]),
+    "pqn_env_reset_params": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_int64, POINTER(EnvParams), c_int,
+                                     c_void_p]),
     "pqn_env_step": (c_int, [c_int, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p, c_void_p,
                              c_void_p, c_void_p, c_void_p, c_int64, c_int, c_int, c_void_p]),
     "pqn_env_obs_packed": (c_int, [c_int, c_void_p, c_void_p, c_int64, c_void_p]),

@@ -27,6 +27,7 @@ enum EnvId : int {
   ENV_SEAQUEST = 4,
   ENV_CARTPOLE = 16,
   ENV_ACROBOT = 17,
+  ENV_MEMORY_CHAIN = 32,
 };
 
 constexpr int LOG_WORDS = 5;

@@ -16,6 +16,7 @@
 #include "../../include/pqn_b200.h"
 #include "api_common.h"
 #include "env_breakout.cuh"
+#include "env_bsuite.cuh"
 #include "env_classic.cuh"
 #include "env_minatar_more.cuh"
 #include "rollout_logic.cuh"
@@ -103,13 +104,14 @@ template <class Env>
 __global__ void __launch_bounds__(ENV_BLOCK) env_reset_kernel(const uint32_t* __restrict__ keys,
                                                               uint32_t* __restrict__ state,
                                                               float* __restrict__ obs, int64_t N, int max_steps,
-                                                              int part) {
+                                                              int memory_length, int part) {
   __shared__ uint32_t smem[ObsScratch<Env>::WORDS];
   const int64_t i = (int64_t)blockIdx.x * ENV_BLOCK + threadIdx.x;
   const bool active = i < N;
   typename Env::State s;
   if (active) {
     Key k{keys[2 * i], keys[2 * i + 1]};
+    env_set_params<Env>(s, memory_length);
     Env::reset_env(k, part, max_steps, s);
     Env::store(s, state, N, i);
     LogState lg;
@@ -357,10 +359,32 @@ static void fill_info(pqn_env_info_t* o) {
     case ENV_SPACE_INVADERS: { using EnvT = SpaceInvadersEnv; __VA_ARGS__; } break; \
     case ENV_CARTPOLE: { using EnvT = CartPoleEnv; __VA_ARGS__; } break;        \
     case ENV_ACROBOT: { using EnvT = AcrobotEnv; __VA_ARGS__; } break;          \
+    case ENV_MEMORY_CHAIN: { using EnvT = MemoryChainEnv; __VA_ARGS__; } break; \
     default: return set_error(PQN_E_UNSUPPORTED, "env id %d is not built into libpqn_b200", env_id); \
   }
 
 static inline unsigned blocks_for(int64_t n, int bs) { return (unsigned)((n + bs - 1) / bs); }
+
+template <class Env>
+static int memory_length_or_default(int memory_length) {
+  if constexpr (EnvHasMemoryLength<Env>::value) return memory_length > 0 ? memory_length : Env::DEFAULT_MEMORY_LENGTH;
+  return 0;
+}
+
+// LogWrapper(env).reset over N envs.  params.max_steps <= 0 selects the env default; so does
+// params.memory_length <= 0 (pqn_env_reset_params rejects that before it gets here).
+static int env_reset(int env_id, const uint32_t* keys, uint32_t* state, float* obs, int64_t N,
+                     pqn_env_params_t params, int rng_mode, void* stream, const char* what) {
+  if (N == 0) return PQN_OK;
+  if (!keys || !state || N < 0) return set_error(PQN_E_INVALID, "%s: bad argument", what);
+  PQN_ENV_DISPATCH(env_id, {
+    const int ms = params.max_steps > 0 ? params.max_steps : EnvT::DEFAULT_MAX_STEPS;
+    const int ml = memory_length_or_default<EnvT>(params.memory_length);
+    { LaunchScope _ls(K_ENV_RESET, (cudaStream_t)stream); env_reset_kernel<EnvT><<<blocks_for(N, ENV_BLOCK), ENV_BLOCK, 0, (cudaStream_t)stream>>>(keys, state, obs, N,
+                                                                                             ms, ml, rng_mode); }
+  });
+  return check_launch(what);
+}
 
 }  // namespace pqn
 
@@ -398,14 +422,18 @@ int pqn_threefry2x32(const uint32_t* key_pairs, const uint32_t* ctr_pairs, uint3
 
 int pqn_env_reset(int env_id, const uint32_t* keys, uint32_t* state, float* obs, int64_t N, int max_steps,
                   int rng_mode, void* stream) {
-  if (N == 0) return PQN_OK;
-  if (!keys || !state || N < 0) return set_error(PQN_E_INVALID, "pqn_env_reset: bad argument");
-  PQN_ENV_DISPATCH(env_id, {
-    const int ms = max_steps > 0 ? max_steps : EnvT::DEFAULT_MAX_STEPS;
-    { LaunchScope _ls(K_ENV_RESET, (cudaStream_t)stream); env_reset_kernel<EnvT><<<blocks_for(N, ENV_BLOCK), ENV_BLOCK, 0, (cudaStream_t)stream>>>(keys, state, obs, N,
-                                                                                             ms, rng_mode); }
-  });
-  return check_launch("pqn_env_reset");
+  const pqn_env_params_t defaults = {max_steps, 0};
+  return env_reset(env_id, keys, state, obs, N, defaults, rng_mode, stream, "pqn_env_reset");
+}
+
+int pqn_env_reset_params(int env_id, const uint32_t* keys, uint32_t* state, float* obs, int64_t N,
+                         const pqn_env_params_t* params_host, int rng_mode, void* stream) {
+  if (!params_host) return set_error(PQN_E_INVALID, "pqn_env_reset_params: params_host is NULL");
+  bool has_memory_length = false;
+  PQN_ENV_DISPATCH(env_id, has_memory_length = EnvHasMemoryLength<EnvT>::value);
+  if (has_memory_length && params_host->memory_length < 1)
+    return set_error(PQN_E_INVALID, "pqn_env_reset_params: memory_length=%d, must be >= 1", params_host->memory_length);
+  return env_reset(env_id, keys, state, obs, N, *params_host, rng_mode, stream, "pqn_env_reset_params");
 }
 
 int pqn_env_step(int env_id, const uint32_t* keys, uint32_t* state, const int32_t* action, float* obs,

@@ -2,9 +2,23 @@
 // CPU logic harness used in tests (tests/host_harness.cpp compiles these same
 // inline functions with g++; the product never runs them on the host).
 #pragma once
+#include <type_traits>
+
 #include "env_common.cuh"
 
 namespace pqn {
+
+// Env parameters beyond max_steps (MemoryChain's memory_length) live in the env's state words.  An env that has one
+// declares set_memory_length(State&, int); env_set_params writes it before reset_env, which leaves it unchanged.
+template <class Env, class = void>
+struct EnvHasMemoryLength : std::false_type {};
+template <class Env>
+struct EnvHasMemoryLength<Env, std::void_t<decltype(&Env::set_memory_length)>> : std::true_type {};
+
+template <class Env>
+PQN_HD void env_set_params(typename Env::State& s, int memory_length) {
+  if constexpr (EnvHasMemoryLength<Env>::value) Env::set_memory_length(s, memory_length);
+}
 
 // gymnax Environment.step (auto-reset) + LogWrapper.step for one env.
 template <class Env>

@@ -21,7 +21,7 @@ from .networks import NET_RNN, QNetworkSpec
 
 
 class PQNRnnEngine:
-    def __init__(self, config: dict, device=None):
+    def __init__(self, config: dict, device=None, env_params: envs.EnvParams | None = None):
         self.cfg = c = config
         self.device = torch.device(device or "cuda")
         if self.device.type != "cuda" or not torch.cuda.is_available():
@@ -32,6 +32,8 @@ class PQNRnnEngine:
                                       "(the shipped pqn_rnn_cartpole.yaml)")
         self.rng_mode = int(c.get("JAX_THREEFRY_PARTITIONABLE", 0))
         self.env, self.env_params = envs.make(c["ENV_NAME"], flatten_obs=True, rng_mode=self.rng_mode)
+        if env_params is not None:                                    # e.g. MemoryChain's memory_length (:134-136)
+            self.env_params = env_params
         if self.env.binary_obs:
             raise NotImplementedError("the recurrent script is built for the classic-control envs")
         self.max_steps = int(self.env_params.max_steps_in_episode)
@@ -69,13 +71,13 @@ class PQNRnnEngine:
                                           _lib.stream_ptr()), "pqn_rollout_act_step")
 
     def _reset(self, key, S, N):
-        """vmap_reset(N)(key): obs [S,N,D], state."""
-        dev, mode = self.device, self.rng_mode
+        """vmap_reset(N)(key, env_params): obs [S,N,D], state."""
+        dev, mode, L = self.device, self.rng_mode, _lib.lib()
         state = torch.empty((self.env.state_words, S * N), dtype=torch.int32, device=dev)
         obs = torch.empty((S, N, self.D), dtype=torch.float32, device=dev)
-        _lib.check(_lib.lib().pqn_env_reset(self.env.env_id, _lib.p(jr.split(key, N, mode).reshape(S * N, 2).contiguous()),
-                                            _lib.p(state), _lib.p(obs), S * N, self.max_steps, mode, _lib.stream_ptr()),
-                   "pqn_env_reset")
+        _lib.check(L.pqn_env_reset_params(self.env.env_id, _lib.p(jr.split(key, N, mode).reshape(S * N, 2).contiguous()),
+                                          _lib.p(state), _lib.p(obs), S * N, envs.c_params(self.env_params), mode,
+                                          _lib.stream_ptr()), "pqn_env_reset_params")
         return obs, state
 
     # ------------------------------------------------------------------ #

@@ -17,7 +17,8 @@ names for interop and parity tests (pure tensor ops, usable on CPU tensors).
 """
 from __future__ import annotations
 
-from dataclasses import dataclass
+import numbers
+from dataclasses import dataclass, replace
 from types import SimpleNamespace
 
 import torch
@@ -31,6 +32,7 @@ ENV_IDS = {
     "Freeway-MinAtar": 3,
     "CartPole-v1": 16,
     "Acrobot-v1": 17,
+    "MemoryChain-bsuite": 32,
 }
 # PQN_ENV_SEAQUEST (4) is reserved in include/pqn_b200.h but not built: gymnax 0.0.6 (the reference's pin) does not
 # register "Seaquest-MinAtar" in gymnax.make either (DESIGN.md section 8), so the reference cannot run it.
@@ -40,9 +42,22 @@ LOG_FIELDS = ("episode_returns", "episode_lengths", "returned_episode_returns",
               "returned_episode_lengths", "timestep")
 
 
+# gymnax memory_chain.EnvParams().memory_length; the library's pqn_env_reset uses the same default
+MEMORY_CHAIN_DEFAULT_MEMORY_LENGTH = 5
+
+
 @dataclass
 class EnvParams:
     max_steps_in_episode: int
+    memory_length: int | None = None      # MemoryChain-bsuite only
+
+
+def _check_memory_length(v):
+    """memory_length as an int >= 1 (a config may hand over 100 or 100.0).  Episodes are memory_length + 1 steps:
+    the context is shown at step 0 and the answer is scored at step memory_length, so 0 has no episode to play."""
+    if isinstance(v, bool) or not isinstance(v, numbers.Real) or not float(v).is_integer() or not 1 <= v < 2 ** 31:
+        raise ValueError(f"MemoryChain-bsuite: memory_length must be an integer in [1, 2^31), got {v!r}")
+    return int(v)
 
 
 def _u2f(t):
@@ -137,6 +152,14 @@ def state_to_fields(env_name: str, state: torch.Tensor) -> dict:
             f[k] = _u2f(st[j])
         f["time"] = st[4]
         core = 5
+    elif env_name == "MemoryChain-bsuite":
+        f["context"] = st[0].unsqueeze(1)                                    # [N, num_bits = 1]
+        f["query"] = st[1]
+        f["total_perfect"] = st[2]
+        f["total_regret"] = st[3]
+        f["time"] = st[4]
+        f["param_memory_length"] = st[5]    # not a gymnax field: the env parameter, kept in the state words
+        core = 6
     else:
         raise KeyError(env_name)
     f["log_episode_returns"] = _u2f(st[core + 0])
@@ -147,8 +170,9 @@ def state_to_fields(env_name: str, state: torch.Tensor) -> dict:
     return f
 
 
-def fields_to_state(env_name: str, f: dict) -> torch.Tensor:
-    """Inverse of :func:`state_to_fields` -> int32[state_words, N]."""
+def fields_to_state(env_name: str, f: dict, params: EnvParams | None = None) -> torch.Tensor:
+    """Inverse of :func:`state_to_fields` -> int32[state_words, N].  MemoryChain's memory_length word comes from
+    ``params`` (gymnax's default when None or unset), not from the gymnax fields."""
     i32 = lambda t: torch.as_tensor(t).to(torch.int32)
     if env_name == "Breakout-MinAtar":
         w = (i32(f["ball_y"]) | (i32(f["ball_x"]) << 4) | (i32(f["ball_dir"]) << 8) | (i32(f["pos"]) << 10)
@@ -207,6 +231,12 @@ def fields_to_state(env_name: str, f: dict) -> torch.Tensor:
     elif env_name == "Acrobot-v1":
         core = [_f2u(torch.as_tensor(f[k])) for k in
                 ("joint_angle1", "joint_angle2", "velocity_1", "velocity_2")] + [i32(f["time"])]
+    elif env_name == "MemoryChain-bsuite":
+        ml = params.memory_length if params is not None and params.memory_length is not None \
+            else MEMORY_CHAIN_DEFAULT_MEMORY_LENGTH
+        t = i32(f["time"])
+        core = [i32(f["context"]).reshape(t.shape[0], -1)[:, 0], i32(f["query"]), i32(f["total_perfect"]),
+                i32(f["total_regret"]), t, torch.full_like(t, _check_memory_length(ml))]
     else:
         raise KeyError(env_name)
     log = [_f2u(torch.as_tensor(f["log_episode_returns"])), i32(f["log_episode_lengths"]),
@@ -253,7 +283,9 @@ class BatchedEnv:
         self.num_actions = info.num_actions
         shape = tuple(info.obs_shape) if self.binary_obs else (info.obs_dim,)
         self._obs_shape = (info.obs_dim,) if flatten_obs else shape
-        self.default_params = EnvParams(max_steps_in_episode=info.max_steps)
+        self.default_params = EnvParams(
+            max_steps_in_episode=info.max_steps,
+            memory_length=MEMORY_CHAIN_DEFAULT_MEMORY_LENGTH if name == "MemoryChain-bsuite" else None)
         self.rng_mode = rng_mode
 
     # gymnax spaces -------------------------------------------------------
@@ -269,9 +301,9 @@ class BatchedEnv:
         n = keys.shape[0]
         state = torch.empty((self.state_words, n), dtype=torch.int32, device=keys.device)
         obs = torch.empty((n,) + self._obs_shape, dtype=torch.float32, device=keys.device)
-        _lib.check(_lib.lib().pqn_env_reset(self.env_id, _lib.p(keys), _lib.p(state), _lib.p(obs), n,
-                                            params.max_steps_in_episode, self.rng_mode, _lib.stream_ptr()),
-                   "pqn_env_reset")
+        _lib.check(_lib.lib().pqn_env_reset_params(self.env_id, _lib.p(keys), _lib.p(state), _lib.p(obs), n,
+                                                   c_params(params), self.rng_mode, _lib.stream_ptr()),
+                   "pqn_env_reset_params")
         return obs, state
 
     def step(self, keys: torch.Tensor, state: torch.Tensor, action: torch.Tensor,
@@ -297,7 +329,25 @@ class BatchedEnv:
         return obs, state, reward, done_b, info
 
 
-def make(env_name: str, flatten_obs: bool = False, rng_mode: int = 0):
-    """``gymnax.make(env_name)`` -> (env, env_params); the LogWrapper is built in."""
+def c_params(params: EnvParams) -> _lib.EnvParams:
+    """EnvParams -> the library's pqn_env_params_t.  memory_length None is passed as 0: envs without the parameter
+    ignore it, MemoryChain rejects it (its params always carry one, see BatchedEnv.default_params)."""
+    ml = params.memory_length
+    return _lib.EnvParams(int(params.max_steps_in_episode), 0 if ml is None else int(ml))
+
+
+def make(env_name: str, flatten_obs: bool = False, rng_mode: int = 0, env_kwargs: dict | None = None):
+    """``gymnax.make(env_name)`` -> (env, env_params); the LogWrapper is built in.
+    ``env_kwargs``: EnvParams fields to override, as ``EnvParams(**env_kwargs)`` would (only MemoryChain-bsuite's
+    ``memory_length`` exists beyond the defaults).  They are validated here, before any device work."""
+    kw = dict(env_kwargs or {})
+    if env_name not in ENV_IDS:
+        raise KeyError(f"unknown env {env_name!r}; known: {sorted(ENV_IDS)}")
+    allowed = {"memory_length"} if env_name == "MemoryChain-bsuite" else set()
+    unknown = set(kw) - allowed
+    if unknown:
+        raise TypeError(f"{env_name}: unknown env parameter(s) {sorted(unknown)}")
+    if "memory_length" in kw:
+        kw["memory_length"] = _check_memory_length(kw["memory_length"])
     env = BatchedEnv(env_name, flatten_obs=flatten_obs, rng_mode=rng_mode)
-    return env, env.default_params
+    return env, replace(env.default_params, **kw)
